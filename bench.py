@@ -3,6 +3,7 @@
 
     python bench.py --gpus 1 --steps K --warmup W [--config c1|c2|c3]   # our arm
     python bench.py --impl reference --gpus 1 ...                       # the reference's CPU path (oracle port) on host cores
+    python bench.py ... --dump-outputs DIR                              # also write the last timed step's outputs as DIR/*.npy
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one frame: clear + project/cull/z-resolve all points into the 4-level packed pyramid, gather the descriptor feature
@@ -44,6 +45,7 @@ C5 = dict(n_points=5_000_000, W=256, H=256, crops_per_gpu=8, depth=250.0,
           workload="train loop: 256x256 random crops (zoom U(0.7,2), shift), 5M points, batch 8 crops per GPU, L1 loss, "
                    "backward through gather + UNet, Adam (net) + RMSprop (descriptors)")
 TOL_BF16, PSNR_BF16 = 3e-2, 45.0             # the stated production-mode tolerance (tests/test_gpu_unet.py, DESIGN.md §2)
+DUMP_LIMIT_BYTES = 64 << 20
 
 
 def metric_name(cfg):
@@ -110,6 +112,19 @@ class ClockSampler:
                     reasons.add(n)
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "samples": len(sm), "reasons": sorted(reasons)}
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: write each array (name -> numpy array) as out_dir/<name>.npy, float64 kept, everything else as float32,
+    so that two builds run with the same arguments can be compared output for output."""
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    arrays = {k: a if a.dtype == np.float64 else a.astype(np.float32) for k, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench.py --dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT_BYTES} byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def psnr(a, b):
@@ -225,7 +240,7 @@ def run_reference_arm(args):
         warm_done += 1
     ts, info = [], None
     for _ in range(max(1, args.steps)):
-        t, info, _, _ = cpu_reference_frame(cfg, xyz, tex, sd)
+        t, info, _, rgb = cpu_reference_frame(cfg, xyz, tex, sd)
         ts.append(t)
         if time.perf_counter() - t_start + t > budget_s:
             break
@@ -242,6 +257,8 @@ def run_reference_arm(args):
             "cpu_baseline": {"value": fps, "unit": "frames/s", "cores": cores, "cpu": cpu_model(), "kind": "port", "sample": sample,
                              "raster_s": info["raster_s"], "gather_net_s": info["gather_net_s"]},
             "e2e": {"value": fps, "unit": "frames/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"rgb": rgb.numpy()})
     print(json.dumps(line), flush=True)
 
 
@@ -455,6 +472,7 @@ def run_ours(args):
     join_side = (lambda: torch.cuda.current_stream().wait_stream(sfs.side)) if world > 1 else None   # K rasters inside K timed steps
     ms_res = timed(resident_step, args.steps, args.warmup, finish=join_side)
     clocks = sampler.stop() if sampler else None
+    last_rgb = eng.output.clone() if args.dump_outputs and rank == 0 else None   # what step() returned last; the next run overwrites it
     if world == 1:
         pyr.clear()
     for s in range(min(3, args.warmup)):
@@ -730,6 +748,8 @@ def run_ours(args):
             "reference_gpu": ref_gpu,
             "reference_surface": surface,
         }
+        if last_rgb is not None:
+            dump_outputs(args.dump_outputs, {"rgb": last_rgb.cpu().numpy()})
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -789,6 +809,7 @@ def run_train(args):
     tim = {"raster": 0.0, "net_fwd_bwd": 0.0, "join": 0.0, "optim": 0.0}
     ev = lambda: torch.cuda.Event(enable_timing=True)
     marks = []
+    last = [None, None]
 
     def step(m_dev, profile=False):
         e = [ev() for _ in range(5)] if profile else None
@@ -817,6 +838,7 @@ def run_train(args):
         if profile:
             e[4].record()
             marks.append(e)
+        last[:] = [loss, out]
         return loss
 
     def barrier():
@@ -846,6 +868,7 @@ def run_train(args):
     sampler = ClockSampler(local) if rank == 0 else None
     ms_res = timed(lambda s: step(mats_dev[s]))
     clocks = sampler.stop() if sampler else None
+    last_out = [t.detach().clone() for t in last] if args.dump_outputs and rank == 0 else None
     our_launches = ops.launch_count() - launches0
 
     def e2e_step(s):
@@ -901,6 +924,8 @@ def run_train(args):
                              "note": "latency-bound at this size (a few 10^5 touched rows); the comparison that matters is the dense optimizer's time"},
                 "breakdown_ms_per_step": tim,
                 "cpu_baseline": None}
+        if last_out is not None:
+            dump_outputs(args.dump_outputs, {"loss": last_out[0].double().cpu().numpy(), "rgb": last_out[1].cpu().numpy()})
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -919,7 +944,12 @@ def main():
     ap.add_argument("--profile-timed-region", action="store_true",
                     help="cudaProfilerStart/Stop around the timed steps and exit (for ncu --profile-from-start off)")
     ap.add_argument("--layer-times", default=None, help="write per-layer CUDA-event timings (JSON) to this path")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (rank 0's frame 'rgb' "
+                         "[1,3,H,W]; c5: the step's 'loss' and its rendered crops 'rgb' [B,3,H,W])")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.config == "c5":
         if args.impl == "reference":

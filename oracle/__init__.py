@@ -13,15 +13,18 @@ Pieces (each cites the reference file:line it follows):
 
 Parity pinning: the reference has no tests or golden vectors for this path
 (SURVEY.md §4: "parity unpinned" by the reference itself).  We pin the oracle
-with (1) hand-derived known-answer tests, (2) golden fixtures generated in the
-build container by importing the reference's own Python modules from
-/root/reference (tests/golden/make_golden.py, fixtures committed), and (3) on a
-GPU box, the reference ``pcpr`` extension compiled from its own sources into
-``oracle/_ref/``.
+with (1) hand-derived known-answer tests, (2) golden fixtures computed by the
+reference's own Python modules (tests/golden/make_golden.py and
+make_reference_modules.py, fixtures committed), and (3) the index/depth maps the
+reference ``pcpr`` extension, compiled from its own sources into ``oracle/_ref/``,
+rendered on a B200 (tests/golden/make_reference_pcpr.py, fixture committed).
 """
+import atexit
 import ctypes
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -31,22 +34,28 @@ _lib = None
 
 
 def build(force=False):
-    """gcc the C restatement (seconds).  -ffp-contract=off: only explicit fmaf() fuses."""
+    """gcc the C restatement (seconds).  -ffp-contract=off: only explicit fmaf() fuses.  Returns the library's path: in the
+    package, or in a temporary directory when the package directory is read-only and holds no current build."""
+    global _SO
     src = os.path.join(_HERE, "zbuffer.c")
     if (not force) and os.path.exists(_SO) and os.path.getmtime(_SO) >= os.path.getmtime(src):
         return _SO
+    out = _SO
+    if not os.access(_HERE, os.W_OK):
+        tmp = tempfile.mkdtemp(prefix="oracle_zbuffer_")
+        atexit.register(shutil.rmtree, tmp, True)
+        out = os.path.join(tmp, os.path.basename(_SO))
     cmd = ["gcc", "-O2", "-fPIC", "-shared", "-ffp-contract=off", "-fno-fast-math", "-mfma",
-           "-o", _SO, src, "-lm"]
+           "-o", out, src, "-lm"]
     subprocess.check_call(cmd)
+    _SO = out
     return _SO
 
 
 def _load():
     global _lib
     if _lib is None:
-        if not os.path.exists(_SO):
-            build()
-        lib = ctypes.CDLL(_SO)
+        lib = ctypes.CDLL(build())
         f32p = ctypes.POINTER(ctypes.c_float)
         lib.oracle_pcpr_forward.argtypes = [f32p, ctypes.c_int64, f32p, ctypes.c_int, ctypes.c_int,
                                             ctypes.c_int, f32p, f32p]

@@ -1,10 +1,9 @@
 """ORACLE — test infrastructure only.
 
 Plain torch-fp32 (CPU) restatement of the reference's descriptor gather and refinement
-net, driven by the reference's own ``state_dict`` (identical keys), so that it can travel
-to the GPU box where /root/reference does not exist.  Pinned in the build container
-against the imported reference modules (tests/test_oracle_pin_reference.py) and against
-the committed fixtures in tests/golden/ (tests/test_oracle_golden.py).
+net, driven by the reference's own ``state_dict`` (identical keys), so that tests need
+neither the reference nor a GPU.  Pinned to outputs of the reference modules stored in
+tests/golden/ (tests/test_oracle_pin_reference.py, tests/test_oracle_golden.py).
 
 Follows:
   READ/models/texture.py:42-70    PointTexture.forward   -> point_texture()

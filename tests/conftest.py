@@ -8,7 +8,6 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-HAVE_REFERENCE = os.path.isdir("/root/reference/READ")
 
 
 def pytest_configure(config):

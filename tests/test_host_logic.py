@@ -136,3 +136,15 @@ def test_sorted_points_store_is_a_spatially_coherent_permutation():
     with pytest.raises(RuntimeError, match="float"):
         ops.SortedPoints(xyz.double())
     assert ops.SortedPoints(torch.empty((0, 3))).n == 0
+
+
+def test_bench_dump_outputs_writes_float_arrays_within_the_size_limit(tmp_path):
+    import bench
+    rgb = np.arange(6, dtype=np.float16).reshape(1, 2, 3)
+    bench.dump_outputs(str(tmp_path / "d"), {"rgb": rgb, "loss": np.float64(0.25)})
+    got = np.load(tmp_path / "d" / "rgb.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, rgb.astype(np.float32))
+    assert np.load(tmp_path / "d" / "loss.npy").dtype == np.float64
+    with pytest.raises(SystemExit):
+        bench.dump_outputs(str(tmp_path / "e"), {"rgb": np.zeros(bench.DUMP_LIMIT_BYTES // 4 + 1, np.float32)})
+    assert not (tmp_path / "e").exists()

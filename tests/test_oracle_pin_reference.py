@@ -1,31 +1,29 @@
-"""Pin the oracle's torch restatement to the reference's real modules (only where /root/reference exists,
-i.e. in the build container; skipped on the GPU box)."""
-import sys
-import types
-
+"""Pin the oracle's torch restatement and our UNet to the reference's real modules, through what those modules computed
+on seeded inputs (tests/golden/reference_modules.npz, written by tests/golden/make_reference_modules.py)."""
 import numpy as np
 import pytest
 import torch
 
-from conftest import HAVE_REFERENCE
+from conftest import load_golden
 from read_b200 import synth
 
-pytestmark = pytest.mark.skipif(not HAVE_REFERENCE, reason="/root/reference not present")
+
+@pytest.fixture(scope="module")
+def ref(synth_sd):
+    g = load_golden("reference_modules")
+    assert abs(synth.state_dict_checksum(synth_sd) - float(g["sd_checksum"])) < 1e-6 * float(g["sd_checksum"]), \
+        "synthetic weights differ from the ones the fixture was generated with (torch RNG changed?)"
+    return g
 
 
-def _ref():
-    if "/root/reference" not in sys.path:
-        sys.path.insert(0, "/root/reference")
-    sys.modules.setdefault("imageio", types.ModuleType("imageio"))
-    from READ.models.unet import UNet
-    from READ.models.texture import PointTexture
-    from READ.models.compose import NetAndTexture
-    return UNet, PointTexture, NetAndTexture
+def _ref_state_dict(g):
+    """The reference UNet's state_dict layout: zero tensors of its keys, shapes and dtypes."""
+    return {str(k): torch.zeros(tuple(int(d) for d in s if d >= 0), dtype=getattr(torch, str(t)))
+            for k, s, t in zip(g["sd_keys"], g["sd_shapes"], g["sd_dtypes"])}
 
 
-def test_state_dict_keys_identical_to_reference(synth_sd):
-    UNet, _, _ = _ref()
-    ref_sd = UNet().state_dict()
+def test_state_dict_keys_identical_to_reference(synth_sd, ref):
+    ref_sd = _ref_state_dict(ref)
     assert set(ref_sd) == set(synth_sd)
     for k, v in ref_sd.items():
         assert tuple(v.shape) == tuple(synth_sd[k].shape), k
@@ -37,45 +35,36 @@ def test_state_dict_keys_identical_to_reference(synth_sd):
     OurUNet().load_state_dict(ref_sd, strict=True)
 
 
-def test_unet_oracle_equals_reference_module(synth_sd):
+def test_unet_oracle_equals_reference_module(synth_sd, ref):
     from oracle import unet_ref
-    UNet, _, _ = _ref()
-    net = UNet()
-    net.load_state_dict(synth_sd, strict=True)
-    net.eval()
     g = torch.Generator().manual_seed(7)
     H, W = 32, 48
     xs = [torch.rand((2, 8, H >> l, W >> l), generator=g) for l in range(5)]
+    want = torch.from_numpy(ref["unet_out"])
     with torch.no_grad():
-        want = net(*xs)
         got = unet_ref.unet_forward(synth_sd, xs)
     assert float((want - got).abs().max()) < 2e-5
 
 
-def test_gather_oracle_equals_reference_module():
+def test_gather_oracle_equals_reference_module(ref):
     from oracle import unet_ref
-    _, PointTexture, _ = _ref()
     g = torch.Generator().manual_seed(3)
-    tex = PointTexture(8, 500, init_method='rand')
     ids = torch.randint(0, 500, (3, 1, 9, 7), generator=g).float()
-    with torch.no_grad():
-        want = tex(ids)
-    got = unet_ref.point_texture(tex.texture_.detach(), ids)
+    np.testing.assert_array_equal(ids.numpy(), ref["ids"])
+    want = torch.from_numpy(ref["gather_out"])
+    got = unet_ref.point_texture(torch.from_numpy(ref["texture"]), ids)
     assert torch.equal(want, got)
 
 
-def test_training_forward_of_our_unet_equals_reference(synth_sd):
+def test_training_forward_of_our_unet_equals_reference(synth_sd, ref):
     """The library (autograd) path of read_b200.unet.UNet must agree with the reference on CPU."""
-    UNet, _, _ = _ref()
     from read_b200.unet import UNet as OurUNet
-    ref, ours = UNet(), OurUNet()
-    ref.load_state_dict(synth_sd)
+    ours = OurUNet()
     ours.load_state_dict(synth_sd)
-    ref.eval()
     ours.eval()
     g = torch.Generator().manual_seed(11)
     xs = [torch.rand((1, 8, 32 >> l, 32 >> l), generator=g) for l in range(4)]
-    want = ref(*xs)
+    want = torch.from_numpy(ref["train_out"])
     got = ours(*xs)                      # grad enabled -> torch path
     assert float((want - got).abs().max()) < 2e-5
     got.sum().backward()
